@@ -25,13 +25,27 @@ def test_reference_arm_prints_contract_line():
     assert len(r.stdout.strip().splitlines()[-1]) < 1500
 
 
-def test_reference_arm_can_bound_its_sample():
+def test_reference_arm_can_bound_its_sample(tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2",
-                        "--warmup", "0", "--rows", "100000", "--ref-rows", "20000"],
+                        "--warmup", "0", "--rows", "100000", "--ref-rows", "20000", "--dump-outputs", str(tmp_path)],
                        capture_output=True, text=True, cwd=ROOT, timeout=300)
     assert r.returncode == 0, r.stderr
     d = json.loads(r.stdout.strip().splitlines()[-1])
     assert d["steps"] == 2 and "scaled x5" in d["cpu_baseline"]["sample"]
+    # --dump-outputs: the hits of the last timed step (query 1) over the 20000 sampled rows
+    sys.path.insert(0, ROOT)
+    import bench
+    import oracle
+    want_rows, want_d = oracle.search_rows(bench.gen_chunk_numpy(0, 100000)[:20000], bench.gen_queries(64)[1], top_k=10)
+    got_d, got_rows = np.load(tmp_path / "hits_distance.npy"), np.load(tmp_path / "hits_row.npy")
+    assert got_d.dtype == got_rows.dtype == np.float64
+    assert np.array_equal(got_rows, want_rows.astype(np.float64)) and np.allclose(got_d, want_d, rtol=0, atol=1e-6)
+
+
+def test_steps_below_one_are_refused():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                       capture_output=True, text=True, cwd=ROOT, timeout=120)
+    assert r.returncode == 2 and "--steps" in r.stderr
 
 
 def test_reference_arm_non_zero_ranks_exit_quietly():

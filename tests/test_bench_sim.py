@@ -7,6 +7,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,9 +36,11 @@ def _torchrun(n, port, extra, env=None):
                           capture_output=True, text=True, cwd=ROOT, env=e, timeout=600)
 
 
-def test_single_gpu_flow_prints_sides_then_a_complete_headline():
+def test_single_gpu_flow_prints_sides_then_a_complete_headline(tmp_path):
+    side_json, dump = tmp_path / "bench_side.json", tmp_path / "dump"
     r = subprocess.run([sys.executable, SIM, "--gpus", "1"] + SMALL + ["--ivfpq-rows", "20000", "--config2-rows", "20000", "--embed-lines", "3000",
-                                                                        "--embed-vocab", "2000"],
+                                                                        "--embed-vocab", "2000", "--side-json", str(side_json),
+                                                                        "--dump-outputs", str(dump)],
                        capture_output=True, text=True, cwd=ROOT, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     out = _lines(r.stdout)
@@ -51,8 +54,18 @@ def test_single_gpu_flow_prints_sides_then_a_complete_headline():
     assert {"bound", "achieved", "peak", "unit", "frac", "traffic"} <= set(head["roofline"])
     assert {"value", "unit", "cores", "kind", "sample"} <= set(head["cpu_baseline"])
     assert {"batch1024_qps", "config2_1M_us", "config4_100M_qps", "ivfpq_recall", "k3_Mlines_s"} <= set(head["side"])
-    full = json.load(open(os.path.join(ROOT, "bench_side.json")))            # the untrimmed line + every section
+    full = json.load(open(side_json))                                          # the untrimmed line + every section
     assert full["headline"]["tier_stats"]["q8"][0] > 0 and set(full["sides"]) >= {"k1_tiers", "config4_100M"}
+    # --dump-outputs: the hits of the last timed step (warm-up 3 + 5 steps -> query 7) over the generated corpus
+    sys.path.insert(0, ROOT)
+    import bench
+    import oracle
+    import torch
+    rows = bench.gen_chunk_torch(torch, torch.device("cpu"), 0, 30000).numpy()
+    want_rows, want_d = oracle.search_rows(rows, bench.gen_queries(64)[7], top_k=10)
+    got_d, got_rows = np.load(dump / "hits_distance.npy"), np.load(dump / "hits_row.npy")
+    assert got_d.dtype == got_rows.dtype == np.float64
+    assert np.array_equal(got_rows, want_rows.astype(np.float64)) and np.array_equal(got_d, want_d)
 
 
 def test_two_rank_flow_runs_the_sharded_sections_in_order():
