@@ -299,6 +299,8 @@ int stb_corpus_destroy(stb_corpus *c) {
   cudaFree(c->shadow);
   cudaFree(c->q8);
   cudaFree(c->q8_scale);
+  cudaFree(c->q4);
+  cudaFree(c->q4_sr);
   cudaFree(c->rows);
   cudaGetLastError();
   delete c;
@@ -313,6 +315,7 @@ static void corpus_changed(stb_corpus *c, bool appended_only = false) {
   c->searches_since_change = 0;
   memset(c->tier_tries, 0, sizeof(c->tier_tries));
   memset(c->tier_proven, 0, sizeof(c->tier_proven));
+  c->coarse_tries = c->coarse_proven = 0;
 }
 
 static int corpus_append_impl(stb_corpus *c, const float *rows, uint64_t n, cudaMemcpyKind kind) {
@@ -438,6 +441,17 @@ static int stb_env_max_tier() {
 // STB_SCAN_OVERLAP=1 (opt-in until timed on hardware): the asynchronous entry points (stb_search_topk_dev,
 // stb_search_topk_xchg, stb_search_many) use the overlapped launch mode (one CTA per SM, dependent released
 // at kernel start); default: they launch like the synchronous ones (full grid, dependent released after the scan).
+// STB_Q8_COARSE=0: no 4-bit coarse stage in front of the q8 scan.  Read per call like STB_SCAN_TIER, so
+// one process can compare the two; results are identical either way.
+static bool stb_env_coarse() {
+  const char *e = getenv("STB_Q8_COARSE");
+  return !(e && e[0] == '0');
+}
+// a reduced-width stage that proves fewer than half of its results on this corpus is skipped
+static bool stage_keeps_failing(uint32_t tries, uint32_t proven) { return tries >= 8 && 2 * proven < tries; }
+static bool coarse_usable(const stb_corpus *c) {
+  return stb_env_coarse() && c->q4 && !stage_keeps_failing(c->coarse_tries, c->coarse_proven);
+}
 static bool stb_env_overlap() {
   const char *e = getenv("STB_SCAN_OVERLAP");
   return e && e[0] == '1';
@@ -448,7 +462,8 @@ static bool stb_env_direct_out() {
 }
 static int best_built_tier(const stb_corpus *c, uint32_t top_k) {
   const int max_tier = stb_env_max_tier();
-  if (max_tier >= STB_TIER_Q8 && top_k <= STB_Q8_MAX_K && c->q8 && c->q8_rows == c->n && !c->q8_bad) return STB_TIER_Q8;
+  if (max_tier >= STB_TIER_Q8 && top_k <= STB_Q8_MAX_K && c->q8 && c->q8_rows == c->n && !c->q8_bad)
+    return coarse_usable(c) ? STB_TIER_Q4Q8 : STB_TIER_Q8;
   if (max_tier >= STB_TIER_H16 && c->shadow && c->shadow_rows == c->n && !c->shadow_bad) return STB_TIER_H16;
   return STB_TIER_F32;
 }
@@ -570,7 +585,7 @@ int stb_search(stb_ctx *ctx, const stb_corpus *corpus, const float *q, uint32_t 
       STB_CUDA(cudaStreamSynchronize(ctx->stream));
       return STB_OK;
     };
-    // Tier ladder: q8 (260 B/row) -> h16 (512 B/row) -> f32 (1 KiB/row).  Every tier ends in the
+    // Tier ladder: coarse + q8 (136 B/row + a few q8 rows) -> q8 (260 B/row) -> h16 (512 B/row) -> f32 (1 KiB/row).  Every tier ends in the
     // same exact f64 re-rank and proves its own result; one that cannot is retried one tier up, so
     // the answer is the oracle's whichever tier produced it.  Reduced-width copies are used when
     // they exist (stb_corpus_prepare) and built lazily from the second query on an unchanged
@@ -584,7 +599,7 @@ int stb_search(stb_ctx *ctx, const stb_corpus *corpus, const float *q, uint32_t 
     for (int tier = STB_TIER_Q8; tier >= STB_TIER_H16 && !proven; --tier) {
       if (tier > max_tier) continue;
       if (tier == STB_TIER_Q8 && top_k > STB_Q8_MAX_K) continue;
-      if (cm->tier_tries[tier] >= 8 && 2 * cm->tier_proven[tier] < cm->tier_tries[tier]) continue;
+      if (stage_keeps_failing(cm->tier_tries[tier], cm->tier_proven[tier])) continue;
       const bool built = (tier == STB_TIER_Q8) ? (cm->q8 && cm->q8_rows == cm->n) : (cm->shadow && cm->shadow_rows == cm->n);
       // a copy that covers a prefix (rows were appended since) is extended right away: converting the
       // new rows costs far less than scanning everything at 1 KiB/row
@@ -593,6 +608,14 @@ int stb_search(stb_ctx *ctx, const stb_corpus *corpus, const float *q, uint32_t 
       const int src = (tier == STB_TIER_Q8) ? corpus_ensure_q8(ctx, cm) : corpus_ensure_shadow(ctx, cm);
       if (src == STB_ERR_STATE) continue;                  // rows that cannot be normalised in fp32
       if (src != STB_OK) return src;
+      if (tier == STB_TIER_Q8 && coarse_usable(cm)) {
+        // the coarse stage is part of the q8 tier: a proven result counts there, an unproven one is
+        // retried by the single-stage q8 scan and counts only against the coarse stage
+        if ((rc = run_fast(STB_TIER_Q4Q8)) != STB_OK) return rc;
+        proven = ctx->status_pin[1] != 0;
+        cm->coarse_tries++;
+        if (proven) { cm->coarse_proven++; cm->tier_tries[tier]++; cm->tier_proven[tier]++; continue; }
+      }
       if ((rc = run_fast(tier)) != STB_OK) return rc;
       proven = ctx->status_pin[1] != 0;
       cm->tier_tries[tier]++;
@@ -905,23 +928,34 @@ static int corpus_ensure_q8(stb_ctx *ctx, stb_corpus *c) {
   }
   uint64_t first = (c->q8 && c->q8_rows < c->n && !c->q8_bad) ? c->q8_rows : 0;      // valid prefix: convert only the new rows
   if (c->n > c->q8_cap_rows || !c->q8) {
-    uint8_t *np = nullptr;
+    // the int8 copy (260 B/row) and the coarse copy in front of it (136 B/row) live and grow together
+    uint8_t *np = nullptr, *n4 = nullptr;
     float *ns = nullptr;
+    float2 *n4s = nullptr;
     const uint64_t cap = std::max<uint64_t>(c->n, c->capacity);
     cudaError_t e = cudaMalloc((void **)&np, cap * 256ull);
     if (e == cudaSuccess) e = cudaMalloc((void **)&ns, cap * sizeof(float));
-    if (e != cudaSuccess) { cudaGetLastError(); cudaFree(np); stb_set_error("q8 tier: cannot allocate %llu MiB", (unsigned long long)(cap * 260 >> 20)); return STB_ERR_NOMEM; }
+    if (e == cudaSuccess) e = cudaMalloc((void **)&n4, cap * 128ull);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&n4s, cap * sizeof(float2));
+    if (e != cudaSuccess) {
+      cudaGetLastError(); cudaFree(np); cudaFree(ns); cudaFree(n4);
+      stb_set_error("q8 tier: cannot allocate %llu MiB", (unsigned long long)(cap * 396 >> 20));
+      return STB_ERR_NOMEM;
+    }
     if (c->q8 && first) {
       STB_CUDA(cudaMemcpyAsync(np, c->q8, first * 256ull, cudaMemcpyDeviceToDevice, ctx->stream));
       STB_CUDA(cudaMemcpyAsync(ns, c->q8_scale, first * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
+      STB_CUDA(cudaMemcpyAsync(n4, c->q4, first * 128ull, cudaMemcpyDeviceToDevice, ctx->stream));
+      STB_CUDA(cudaMemcpyAsync(n4s, c->q4_sr, first * sizeof(float2), cudaMemcpyDeviceToDevice, ctx->stream));
       STB_CUDA(cudaStreamSynchronize(ctx->stream));
     } else first = 0;
-    cudaFree(c->q8); cudaFree(c->q8_scale);
-    c->q8 = np; c->q8_scale = ns; c->q8_cap_rows = cap;
+    cudaFree(c->q8); cudaFree(c->q8_scale); cudaFree(c->q4); cudaFree(c->q4_sr);
+    c->q8 = np; c->q8_scale = ns; c->q4 = n4; c->q4_sr = n4s; c->q8_cap_rows = cap;
   }
   int rc;
   STB_CUDA(cudaMemsetAsync(ctx->err_flag, 0, sizeof(int), ctx->stream));
   if ((rc = stb_launch_q8_build(ctx, c->rows, first, c->n, c->q8, c->q8_scale, ctx->err_flag)) != STB_OK) return rc;
+  if ((rc = stb_launch_q4_build(ctx, c->rows, first, c->n, c->q4, c->q4_sr, ctx->err_flag)) != STB_OK) return rc;
   int flag = 0;
   STB_CUDA(cudaMemcpyAsync(&flag, ctx->err_flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   STB_CUDA(cudaMemsetAsync(ctx->err_flag, 0, sizeof(int), ctx->stream));

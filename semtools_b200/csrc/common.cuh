@@ -45,6 +45,9 @@
 #define STB_TIER_F32 0
 #define STB_TIER_H16 1
 #define STB_TIER_Q8 2
+// Not a tier of its own: a 4-bit coarse pass (136 B/row) whose candidates each CTA re-scores with the
+// q8 copy; built and invalidated with q8, counted and reported as q8 (scan_topk.cu: stb_scan_q4).
+#define STB_TIER_Q4Q8 3
 // q8 scores are upper bounds of the exact cosine up to the fp32 evaluation of the bound itself
 // and of the two normalisations (< 4e-6, scan_topk.cu: stb_scan_q8); proof slack:
 #define STB_Q8_SCAN_EPS 2.0e-5
@@ -189,9 +192,13 @@ struct stb_corpus {
   uint64_t q8_rows;          // rows covered (== n when valid)
   uint64_t q8_cap_rows;
   int q8_bad;
+  // coarse copy in front of q8 (same rows, capacity and bad flag): 4-bit codes [capacity][128] + (s4, r)
+  uint8_t *q4;
+  float2 *q4_sr;
   // per-tier bookkeeping: a reduced-width tier is skipped once it proves fewer than half of its
   // results on this corpus (index = STB_TIER_*)
   uint32_t tier_tries[3], tier_proven[3];
+  uint32_t coarse_tries, coarse_proven;   // the same rule for the coarse stage in front of q8
   uint32_t searches_since_change;   // lazy builds wait for the second query on an unchanged corpus
 };
 
@@ -199,7 +206,7 @@ struct stb_corpus {
 // Fast path: one kernel = scan + per-warp running top-K' + CTA/tree merge +
 // exact f64 re-rank + completeness check.  q_dev: 256 f32 on device.
 // n_ranges > 0: ranges_dev holds local [begin,end,vstart] triples.
-// tier: STB_TIER_* -- which copy of `c` the streaming pass reads (must exist and be current).
+// tier: STB_TIER_* or STB_TIER_Q4Q8 -- which copy of `c` the streaming pass reads (must exist and be current).
 // overlapped: the launch is one of a pipelined series (asynchronous entry points): the grid is sized
 // for ONE CTA per SM and releases its dependent at its START, so the next query's scan co-runs with
 // this one instead of waiting for it to drain (scan_topk.cu: "overlapped launches").
@@ -210,6 +217,9 @@ int stb_launch_scan_topk(stb_ctx *ctx, const stb_corpus *c, int tier, const floa
 // int8 codes + scales of rows [first_row, n_rows) (q8 tier)
 int stb_launch_q8_build(stb_ctx *ctx, const float *rows_dev, uint64_t first_row, uint64_t n_rows, uint8_t *out,
                         float *scale, int *bad_flag_dev);
+// 4-bit codes + (s4, r) of rows [first_row, n_rows) (coarse stage in front of q8)
+int stb_launch_q4_build(stb_ctx *ctx, const float *rows_dev, uint64_t first_row, uint64_t n_rows, uint8_t *out,
+                        float2 *sr, int *bad_flag_dev);
 // Largest top_k the fast path serves.
 uint32_t stb_scan_topk_max_k(void);
 // Collect path: every row whose approximate cosine >= cos_floor (or that cannot be

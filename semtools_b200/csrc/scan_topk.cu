@@ -346,16 +346,8 @@ __device__ __forceinline__ void stb_scan_shadow(const ScanArgs &args, const uint
 // term folded into the score, so rows with a large scale are promoted instead of widening a
 // global margin.  A zero or unscorable query makes every score +inf: the proof fails and the
 // caller falls through to the f32 tiers.
-template <int U, int RANGES, class Sink>
-__device__ __forceinline__ void stb_scan_q8(const ScanArgs &args, const uint8_t *q8, const float *q8_scale, Sink &sink) {
-  const int lane = threadIdx.x & 31;
-  const int g = lane >> 3;   // row group inside the warp
-  const int j = lane & 7;    // this lane reads row bytes [16j, 16j+16) and [128+16j, 128+16j+16)
-  float4 q[8];
-  const float4 *q4 = reinterpret_cast<const float4 *>(args.q);
-#pragma unroll
-  for (int i = 0; i < 4; ++i) { q[i] = __ldg(q4 + 4 * j + i); q[4 + i] = __ldg(q4 + 32 + 4 * j + i); }
-  const StbQueryNorm qn = stb_query_norm(q);
+// max |q^_i| of the lane's 8 float4 (the 8 lanes of a group hold the whole query)
+__device__ __forceinline__ float stb_query_amax(const float4 (&q)[8], float rq) {
   float amax = 0.f;
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
@@ -364,34 +356,74 @@ __device__ __forceinline__ void stb_scan_q8(const ScanArgs &args, const uint8_t 
   amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, 4));
   amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, 2));
   amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, 1));
-  amax *= qn.rq;                                            // max |q^_i|
-  const bool q_unusable = qn.q_zero || qn.q_bad || !(amax > 0.f && amax <= 1.0001f);
-  const float S = q_unusable ? 1.f : 32639.0f / amax;
-  const float qs = qn.rq * S;
-  uint32_t qhi[8], qlo[8];
-  int l1 = 0;
+  return amax * rq;
+}
+
+// The q8 tier's query side for lane j of a row group: q16 split into two signed bytes for the row
+// bytes [16j, 16j+16) and [128+16j, 128+16j+16), plus the terms of the upper bound.  Called by the
+// full warp (group reductions).
+struct StbQ8Query {
+  uint32_t hi[8], lo[8];
+  float inv_S, h_l1, e_q;
+  bool unusable;
+  __device__ __forceinline__ void load(const float *qp, int j) {
+    float4 q[8];
+    const float4 *q4 = reinterpret_cast<const float4 *>(qp);
 #pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const float f[4] = {q[i].x, q[i].y, q[i].z, q[i].w};
-    uint32_t hw = 0, lw = 0;
+    for (int i = 0; i < 4; ++i) { q[i] = __ldg(q4 + 4 * j + i); q[4 + i] = __ldg(q4 + 32 + 4 * j + i); }
+    const StbQueryNorm qn = stb_query_norm(q);
+    const float amax = stb_query_amax(q, qn.rq);            // max |q^_i|
+    unusable = qn.q_zero || qn.q_bad || !(amax > 0.f && amax <= 1.0001f);
+    const float S = unusable ? 1.f : 32639.0f / amax;
+    const float qs = qn.rq * S;
+    int l1 = 0;
 #pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      int v = q_unusable ? 0 : __float2int_rn(f[e] * qs);
-      v = max(-32639, min(32639, v));
-      l1 += abs(v);
-      const int lo = ((v + 128) & 255) - 128;               // signed low byte
-      const int hi = (v - lo) >> 8;                         // exact: v - lo is a multiple of 256
-      hw |= (uint32_t)(hi & 255) << (8 * e);
-      lw |= (uint32_t)(lo & 255) << (8 * e);
+    for (int i = 0; i < 8; ++i) {
+      const float f[4] = {q[i].x, q[i].y, q[i].z, q[i].w};
+      uint32_t hw = 0, lw = 0;
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        int v = unusable ? 0 : __float2int_rn(f[e] * qs);
+        v = max(-32639, min(32639, v));
+        l1 += abs(v);
+        const int l = ((v + 128) & 255) - 128;              // signed low byte
+        const int h = (v - l) >> 8;                         // exact: v - l is a multiple of 256
+        hw |= (uint32_t)(h & 255) << (8 * e);
+        lw |= (uint32_t)(l & 255) << (8 * e);
+      }
+      hi[i] = hw; lo[i] = lw;
     }
-    qhi[i] = hw; qlo[i] = lw;
+    l1 += __shfl_xor_sync(0xffffffffu, l1, 4);
+    l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+    l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
+    inv_S = 1.0f / S;
+    h_l1 = 0.50025f * (float)l1 * inv_S;                    // (0.5 + 3e-5 + fp slack) * ||q~||_1
+    e_q = 9.7f * inv_S;
   }
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 4);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-  const float inv_S = 1.0f / S;
-  const float h_l1 = 0.50025f * (float)l1 * inv_S;          // (0.5 + 3e-5 + fp slack) * ||q~||_1
-  const float e_q = 9.7f * inv_S;
+  // upper bound of the exact cosine of the row whose 32 code bytes this lane holds (full warp: group reduction)
+  __device__ __forceinline__ float bound(const uint4 &a0, const uint4 &a1, float scale) const {
+    int dh = 0, dl = 0;
+    const uint32_t w[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      dh = __dp4a((int)w[i], (int)hi[i], dh);
+      dl = __dp4a((int)w[i], (int)lo[i], dl);
+    }
+    int dot = dh * 256 + dl;
+    dot += __shfl_xor_sync(0xffffffffu, dot, 4);
+    dot += __shfl_xor_sync(0xffffffffu, dot, 2);
+    dot += __shfl_xor_sync(0xffffffffu, dot, 1);
+    return unusable ? CUDART_INF_F : fmaf(scale, fmaf((float)dot, inv_S, h_l1), e_q);
+  }
+};
+
+template <int U, int RANGES, class Sink>
+__device__ __forceinline__ void stb_scan_q8(const ScanArgs &args, const uint8_t *q8, const float *q8_scale, Sink &sink) {
+  const int lane = threadIdx.x & 31;
+  const int g = lane >> 3;   // row group inside the warp
+  const int j = lane & 7;    // this lane reads row bytes [16j, 16j+16) and [128+16j, 128+16j+16)
+  StbQ8Query qq;
+  qq.load(args.q, j);
 
   constexpr uint64_t tile_rows = 4 * U;
   const uint64_t n_tiles = (args.n_virtual + tile_rows - 1) / tile_rows;
@@ -419,18 +451,7 @@ __device__ __forceinline__ void stb_scan_q8(const ScanArgs &args, const uint8_t 
     float sc[U];
 #pragma unroll
     for (int u = 0; u < U; ++u) {
-      int dh = 0, dl = 0;
-      const uint32_t w[8] = {a[u][0].x, a[u][0].y, a[u][0].z, a[u][0].w, a[u][1].x, a[u][1].y, a[u][1].z, a[u][1].w};
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        dh = __dp4a((int)w[i], (int)qhi[i], dh);
-        dl = __dp4a((int)w[i], (int)qlo[i], dl);
-      }
-      int dot = dh * 256 + dl;
-      dot += __shfl_xor_sync(0xffffffffu, dot, 4);
-      dot += __shfl_xor_sync(0xffffffffu, dot, 2);
-      dot += __shfl_xor_sync(0xffffffffu, dot, 1);
-      const float s = q_unusable ? CUDART_INF_F : fmaf(sc_row[u], fmaf((float)dot, inv_S, h_l1), e_q);
+      const float s = qq.bound(a[u][0], a[u][1], sc_row[u]);
       sc[u] = valid[u] ? s : -CUDART_INF_F;
     }
     float s = -CUDART_INF_F;
@@ -440,6 +461,186 @@ __device__ __forceinline__ void stb_scan_q8(const ScanArgs &args, const uint8_t 
       if (j == u) { s = sc[u]; r = row[u]; }
     sink.template consume<4 * U>(s, r);
   });
+}
+
+// Coarse pass in front of the q8 tier ("q4"): a 4-bit copy, 128 B of codes + (s4, r) per row = 136 B.
+// Row model (stb_q4_build_kernel): x~_i = s4 * (c_i - 7.5), c_i in [0, 15] (16 mid-rise levels) on the
+// fp32-normalised row x^, with s4 picked per row to minimise r = ||x^ - x~||_2, stored rounded up.
+// Byte b of the row's 32-bit word l holds c[8l+b] in its low nibble and c[8l+4+b] in its high one, so
+// lane j of a row group reads one 16-byte chunk = elements 32j .. 32j+31, and the query, quantised per
+// call to int8 (q8_i = rint(q^_i * S8), S8 = 127 / max|q^_i|), lines up byte for byte with the two
+// nibble planes: two masks, one shift and two dp4a per word, exact in int32.  With q~ = q8 / S8 and
+// f = q^ - q~, Cauchy-Schwarz gives for the exact cosine c = q^ . x^:
+//     c = q~ . x~ + q~ . (x^ - x~) + f . x^  <=  q~ . x~ + r (1 + ||f||) + ||f||
+//     q~ . x~ = s4 * (2 dot - 15 sum(q8)) / (2 S8)          (integer part exact)
+//     u4 = s4 * (2 dot - 15 sum(q8)) / (2 S8) + r (1 + ||f||) + ||f|| + 4e-6   >=  c - 1e-5
+// (||f|| is evaluated in fp32 and inflated; the fp32 normalisations of row and query stay inside the
+// 1e-5, as for q8).  u4 is ~0.1 wide against q8's ~0.01, so it only ranks: the warps keep their best
+// 64 by u4, the CTA re-scores the few that can matter with the q8 codes (stb_scan_topk_kernel, SRC 3)
+// and the tree above sees q8 bounds only.
+template <int U, int RANGES, class Sink>
+__device__ __forceinline__ void stb_scan_q4(const ScanArgs &args, const uint8_t *q4, const float2 *q4_sr, Sink &sink) {
+  static_assert(U % 8 == 0, "a lane carries rows u = j + 8h to the sink");
+  const int lane = threadIdx.x & 31;
+  const int g = lane >> 3;   // row group inside the warp
+  const int j = lane & 7;    // this lane reads row bytes [16j, 16j+16) = elements 32j .. 32j+31
+  float4 q[8];
+  const float4 *qf4 = reinterpret_cast<const float4 *>(args.q);
+#pragma unroll
+  for (int i = 0; i < 8; ++i) q[i] = __ldg(qf4 + 8 * j + i);
+  const StbQueryNorm qn = stb_query_norm(q);
+  const float amax = stb_query_amax(q, qn.rq);
+  const bool q_unusable = qn.q_zero || qn.q_bad || !(amax > 0.f && amax <= 1.0001f);
+  const float S = q_unusable ? 1.f : 127.0f / amax;
+  const float qs = qn.rq * S, inv_S = 1.0f / S;
+  // qw[2i] pairs with the low nibbles of word i (elements 32j+8i .. +3), qw[2i+1] with the high ones
+  uint32_t qw[8];
+  int qsum = 0;
+  float f2 = 0.f;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    const float f[4] = {q[i].x, q[i].y, q[i].z, q[i].w};
+    uint32_t w = 0;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      int v = q_unusable ? 0 : __float2int_rn(f[e] * qs);
+      v = max(-127, min(127, v));
+      qsum += v;
+      const float d = fmaf(-(float)v, inv_S, f[e] * qn.rq);   // f_i = q^_i - q~_i
+      f2 = fmaf(d, d, f2);
+      w |= (uint32_t)(v & 255) << (8 * e);
+    }
+    qw[i] = w;
+  }
+  qsum += __shfl_xor_sync(0xffffffffu, qsum, 4);
+  qsum += __shfl_xor_sync(0xffffffffu, qsum, 2);
+  qsum += __shfl_xor_sync(0xffffffffu, qsum, 1);
+  f2 += __shfl_xor_sync(0xffffffffu, f2, 4);
+  f2 += __shfl_xor_sync(0xffffffffu, f2, 2);
+  f2 += __shfl_xor_sync(0xffffffffu, f2, 1);
+  const float nf = sqrtf(f2) * 1.001f + 2e-6f;              // ||f||, rounded up (each f_i is within 1 ulp)
+  const float coef = 0.5f * inv_S;
+  const int qsum15 = 15 * qsum;
+  const float r_mul = 1.0f + nf, slack = nf + 4e-6f;
+
+  constexpr uint64_t tile_rows = 4 * U;
+  const uint64_t n_tiles = (args.n_virtual + tile_rows - 1) / tile_rows;
+  StbRowMap<RANGES> rmap;
+  rmap.restart();
+  stb_for_each_tile<RANGES, 1>(args, n_tiles, [&](uint64_t tile, bool first) {
+    if (first) rmap.restart();
+    uint4 a[U];
+    uint32_t own_row[U / 8];   // the rows this lane hands to the sink: u = j + 8h
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      const uint64_t v = tile * tile_rows + (uint64_t)(u * 4 + g);
+      const uint64_t vc = v < args.n_virtual ? v : (args.n_virtual - 1);
+      const uint32_t row = rmap.map(args, vc);
+      const float4 t = stb_ld_stream(reinterpret_cast<const float4 *>(q4 + (size_t)row * 128 + (size_t)j * 16));
+      a[u] = make_uint4(__float_as_uint(t.x), __float_as_uint(t.y), __float_as_uint(t.z), __float_as_uint(t.w));
+      if ((u & 7) == j) own_row[u >> 3] = row;
+    }
+#pragma unroll
+    for (int h = 0; h < U / 8; ++h) {
+      const float2 sr = __ldg(q4_sr + own_row[h]);
+      int own_dot = 0;
+#pragma unroll
+      for (int uu = 0; uu < 8; ++uu) {
+        const uint4 &w = a[8 * h + uu];
+        const uint32_t ww[4] = {w.x, w.y, w.z, w.w};
+        int d = 0;
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          d = __dp4a((int)(ww[i] & 0x0f0f0f0fu), (int)qw[2 * i], d);
+          d = __dp4a((int)((ww[i] >> 4) & 0x0f0f0f0fu), (int)qw[2 * i + 1], d);
+        }
+        d += __shfl_xor_sync(0xffffffffu, d, 4);
+        d += __shfl_xor_sync(0xffffffffu, d, 2);
+        d += __shfl_xor_sync(0xffffffffu, d, 1);
+        if (uu == j) own_dot = d;
+      }
+      const uint64_t v = tile * tile_rows + (uint64_t)((8 * h + j) * 4 + g);
+      float s = q_unusable ? CUDART_INF_F : fmaf(sr.x * coef, (float)(2 * own_dot - qsum15), fmaf(sr.y, r_mul, slack));
+      if (v >= args.n_virtual) s = -CUDART_INF_F;
+      sink.template consume<32>(s, own_row[h]);
+    }
+  });
+}
+
+// q4 builder: one warp per row, lane l owns elements 8l .. 8l+7 and writes word l of the row's codes.
+// Normalisation and the bad-row flag are stb_q8_build_kernel's.  s4 = t * max|x^| / 7.5 with t from a
+// fixed set: the one with the smallest ||x^ - x~||_2 (fp32, first on ties).  r is that norm for the
+// stored s4 and codes, evaluated in f64 and rounded up to f32 (a proof input).  Zero rows: s4 = r = 0.
+#define STB_Q4_T_STEPS 8
+__global__ void __launch_bounds__(256)
+stb_q4_build_kernel(const float4 *__restrict__ rows, uint64_t first_row, uint64_t n_rows, uint8_t *__restrict__ out,
+                    float2 *__restrict__ sr, int *bad_flag) {
+  const int lane = threadIdx.x & 31;
+  const uint64_t row = first_row + (uint64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+  if (row >= n_rows) return;
+  const float4 v0 = __ldg(rows + row * STB_ROW_F4 + 2 * lane);
+  const float4 v1 = __ldg(rows + row * STB_ROW_F4 + 2 * lane + 1);
+  float ss = v0.x * v0.x + v0.y * v0.y + v0.z * v0.z + v0.w * v0.w + v1.x * v1.x + v1.y * v1.y + v1.z * v1.z + v1.w * v1.w;
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, off);
+  float inv = 0.f;
+  if (ss != 0.f) {
+    if (!(ss >= 1e-30f && ss <= 1e30f)) { if (lane == 0) atomicExch(bad_flag, 1); }   // NaN/inf/extreme
+    else inv = rsqrtf(ss);
+  } else {
+    const bool nz = (v0.x != 0.f) | (v0.y != 0.f) | (v0.z != 0.f) | (v0.w != 0.f) | (v1.x != 0.f) | (v1.y != 0.f) |
+                    (v1.z != 0.f) | (v1.w != 0.f);
+    if (__any_sync(0xffffffffu, nz) && lane == 0) atomicExch(bad_flag, 1);             // underflowed tiny row
+  }
+  const float x[8] = {v0.x * inv, v0.y * inv, v0.z * inv, v0.w * inv, v1.x * inv, v1.y * inv, v1.z * inv, v1.w * inv};
+  float am = 0.f;
+#pragma unroll
+  for (int e = 0; e < 8; ++e) am = fmaxf(am, fabsf(x[e]));
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) am = fmaxf(am, __shfl_xor_sync(0xffffffffu, am, off));
+  auto code = [](float xe, float inv_s) { return max(0, min(15, __float2int_rn(fmaf(xe, inv_s, 7.5f)))); };
+  float s = 0.f, best = CUDART_INF_F;
+  if (am > 0.f) {
+    for (int k = 0; k < STB_Q4_T_STEPS; ++k) {
+      const float sk = (0.65f + 0.05f * (float)k) * am * (1.0f / 7.5f);
+      const float inv_s = 1.0f / sk;
+      float err = 0.f;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float d = x[e] - sk * ((float)code(x[e], inv_s) - 7.5f);
+        err = fmaf(d, d, err);
+      }
+#pragma unroll
+      for (int off = 16; off > 0; off >>= 1) err += __shfl_xor_sync(0xffffffffu, err, off);
+      if (err < best) { best = err; s = sk; }
+    }
+  }
+  const float inv_s = s > 0.f ? 1.0f / s : 0.f;
+  uint32_t w = 0;
+  double e2 = 0.0;
+#pragma unroll
+  for (int e = 0; e < 8; ++e) {
+    const int c = s > 0.f ? code(x[e], inv_s) : 8;
+    w |= (uint32_t)c << (e < 4 ? 8 * e + 0 : 8 * (e - 4) + 4);
+    const double d = (double)x[e] - (double)s * ((double)c - 7.5);   // s * (c - 7.5) is exact in f64
+    e2 = fma(d, d, e2);
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) e2 += __shfl_xor_sync(0xffffffffu, e2, off);
+  reinterpret_cast<uint32_t *>(out + row * 128)[lane] = w;
+  // f64 sum and sqrt are within a few 1e-16 relative: the 1e-9 margin and upward rounding keep r >= the true norm
+  if (lane == 0) sr[row] = make_float2(s, s > 0.f ? __double2float_ru(sqrt(e2) * (1.0 + 1e-9)) : 0.f);
+}
+
+int stb_launch_q4_build(stb_ctx *ctx, const float *rows_dev, uint64_t first_row, uint64_t n_rows, uint8_t *out,
+                        float2 *sr, int *bad_flag_dev) {
+  if (first_row >= n_rows) return STB_OK;
+  const unsigned blocks = (unsigned)((n_rows - first_row + 7) / 8);
+  stb_q4_build_kernel<<<blocks, 256, 0, ctx->stream>>>(reinterpret_cast<const float4 *>(rows_dev), first_row, n_rows, out, sr,
+                                                       bad_flag_dev);
+  STB_CUDA(cudaGetLastError());
+  ctx->kernel_launches++;
+  return STB_OK;
 }
 
 // q8 builder: one warp per row; lane l owns elements 8l .. 8l+7.  Rows whose fp32 squared norm
@@ -608,9 +809,47 @@ struct TopkArgs {
   unsigned long long *dbg;   // STB_TAIL_TIMING builds only: phase timestamps (ns)
   const uint8_t *shadow;     // SRC == 1: 16-bit normalised corpus shadow (UMMA tile layout)
   uint32_t early_trigger;    // overlapped launch: release the dependent launch at kernel start
-  const uint8_t *q8;         // SRC == 2: int8 codes [n][256] ...
-  const float *q8_scale;     //           ... and per-row scales [n]
+  const uint8_t *q8;         // SRC == 2, 3: int8 codes [n][256] ...
+  const float *q8_scale;     //              ... and per-row scales [n]
+  const uint8_t *q4;         // SRC == 3: 4-bit codes [n][128] ...
+  const float2 *q4_sr;       //           ... and per-row (s4, r) [n]
 };
+
+// SRC 3, after the scan: the CTA's coarse candidates sit in keys[0, c) as (u4, row).  Each is re-scored
+// with the q8 codes (StbQ8Query::bound) and its key replaced by min(u4, u8) -- both are upper bounds of
+// the exact cosine.  32 row groups of 8 lanes, 4 rows per group per pass (<= 512 candidates).
+__device__ __forceinline__ void stb_q8_refine(const TopkArgs &args, uint64_t *keys, int c) {
+  constexpr int R = 4;
+  const int grp = threadIdx.x >> 3, j = threadIdx.x & 7;
+  StbQ8Query qq;
+  qq.load(args.scan.q, j);
+  for (int base = 0; base < c; base += 32 * R) {           // c is CTA-uniform
+    uint4 a[R][2];
+    float sc[R];
+#pragma unroll
+    for (int u = 0; u < R; ++u) {
+      const int idx = base + grp + 32 * u;
+      a[u][0] = a[u][1] = make_uint4(0u, 0u, 0u, 0u);
+      sc[u] = 0.f;
+      if (idx < c) {
+        const uint32_t row = stb_key_row(keys[idx]);
+        const uint4 *p = reinterpret_cast<const uint4 *>(args.q8 + (size_t)row * 256 + (size_t)j * 16);
+        a[u][0] = __ldg(p);
+        a[u][1] = __ldg(p + 8);
+        sc[u] = __ldg(args.q8_scale + row);
+      }
+    }
+#pragma unroll
+    for (int u = 0; u < R; ++u) {
+      const int idx = base + grp + 32 * u;
+      const float u8 = qq.bound(a[u][0], a[u][1], sc[u]);
+      if (idx < c && j == 0) {
+        const uint64_t key = keys[idx];
+        keys[idx] = stb_make_key(fminf(stb_key_score(key), u8), stb_key_row(key));
+      }
+    }
+  }
+}
 
 __device__ __forceinline__ unsigned long long stb_globaltimer() {
   unsigned long long t;
@@ -673,12 +912,17 @@ template <int E, int U, int RANGES, int SRC = 0, int EF = E>
 __global__ void __launch_bounds__(STB_SCAN_THREADS, STB_SCAN_MINB)
 stb_scan_topk_kernel(const TopkArgs args) {
   // SRC 0: scores from the f32 rows; SRC 1: from the 16-bit shadow (wider proof margin);
-  // SRC 2: upper bounds of the exact cosine from the int8 copy (margin folded into the score)
-  constexpr double kScoreEps = SRC == 1 ? STB_SHADOW_SCAN_EPS : (SRC == 2 ? STB_Q8_SCAN_EPS : STB_SCORE_EPS);
+  // SRC 2: upper bounds of the exact cosine from the int8 copy (margin folded into the score);
+  // SRC 3: 4-bit coarse bounds in the warps, re-scored with the int8 copy in the CTA (stb_scan_q4)
+  constexpr double kScoreEps = SRC == 1 ? STB_SHADOW_SCAN_EPS : (SRC >= 2 ? STB_Q8_SCAN_EPS : STB_SCORE_EPS);
+  constexpr uint32_t kTierReported = SRC == 3 ? STB_TIER_Q8 : SRC;   // the status word knows tiers 0..2
+  // SRC 3: the warps rank by the ~0.1-wide 4-bit bound, so their lists are 64 long (room for the rows that
+  // can reach c_k, DESIGN.md section 5); the CTA re-scores them with q8 and publishes KP keys like every tier
+  constexpr int ES = SRC == 3 ? 2 : E;
   constexpr int KP = 32 * E;          // list length below the root
   constexpr int KF = 32 * EF;         // candidates the root keeps
   constexpr int KPS = KP + 1;         // published list stride: KP keys + the node's drop bound
-  static_assert(EF >= E && 8 * KP <= STB_SORT_CAP && KF <= STB_SORT_CAP / 2, "list sizes");
+  static_assert(EF >= E && 8 * 32 * ES <= STB_SORT_CAP && KF <= STB_SORT_CAP / 2, "list sizes");
   __shared__ uint64_t skeys[STB_SORT_CAP];
   __shared__ unsigned int s_T, s_cnt, s_ticket, s_bound, s_nin;
   __shared__ unsigned long long s_T64;
@@ -694,9 +938,10 @@ stb_scan_topk_kernel(const TopkArgs args) {
   // grid leaves HBM idle (CTA merge before exit, launch, ramp-up) are covered by the other scan.
   // Tails stay ordered: everything after the scan sits behind griddepcontrol.wait.
   if (args.early_trigger) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  TopSink<E> sink;
+  TopSink<ES> sink;
   sink.init();
-  if constexpr (SRC == 2) stb_scan_q8<U, RANGES>(args.scan, args.q8, args.q8_scale, sink);
+  if constexpr (SRC == 3) stb_scan_q4<U, RANGES>(args.scan, args.q4, args.q4_sr, sink);
+  else if constexpr (SRC == 2) stb_scan_q8<U, RANGES>(args.scan, args.q8, args.q8_scale, sink);
   else if constexpr (SRC == 1) stb_scan_shadow<U, RANGES>(args.scan, args.shadow, sink);
   else stb_scan_rows<U, RANGES>(args.scan, sink);
   STB_T_MAX(1);                      // last CTA leaves the scan loop
@@ -719,16 +964,21 @@ stb_scan_topk_kernel(const TopkArgs args) {
   {
     const unsigned T = s_T;
 #pragma unroll
-    for (int e = 0; e < E; ++e) {
+    for (int e = 0; e < ES; ++e) {
       const bool take = sink.lr[e] != 0xffffffffu && stb_f2ord(sink.ls[e]) >= T;
       const unsigned m = __ballot_sync(0xffffffffu, take);
       unsigned base = 0u;
-      if (lane == 0 && m) base = atomicAdd(&s_cnt, (unsigned)__popc(m));   // <= 8*KP <= STB_SORT_CAP
+      if (lane == 0 && m) base = atomicAdd(&s_cnt, (unsigned)__popc(m));   // <= 8*32*ES <= STB_SORT_CAP
       base = __shfl_sync(0xffffffffu, base, 0);
       if (take) skeys[base + __popc(m & ((1u << lane) - 1u))] = stb_make_key(sink.ls[e], sink.lr[e]);
     }
   }
   __syncthreads();
+  if constexpr (SRC == 3) {
+    // the keys are u4 bounds so far: T (= T4) covers every row they dropped, the q8 re-score decides the rest
+    stb_q8_refine(args, skeys, (int)s_cnt);
+    __syncthreads();
+  }
   unsigned bound;                                // uniform per CTA from here on
   {
     const int c = (int)s_cnt;
@@ -972,7 +1222,7 @@ stb_scan_topk_kernel(const TopkArgs args) {
       args.out_status[0] = n_out;
       args.out_status[1] = complete ? 1u : 0u;
       args.out_status[2] = (uint32_t)n_valid;
-      args.out_status[3] = (uint32_t)KF | ((uint32_t)SRC << 16);
+      args.out_status[3] = (uint32_t)KF | (kTierReported << 16);
     }
     return;
   }
@@ -1054,7 +1304,7 @@ stb_scan_topk_kernel(const TopkArgs args) {
     args.out_status[0] = min(total, k);
     args.out_status[1] = all_complete;
     args.out_status[2] = s_timeout ? 0xfffffffeu : (uint32_t)n_valid;
-    args.out_status[3] = (uint32_t)KF | ((uint32_t)SRC << 16);
+    args.out_status[3] = (uint32_t)KF | (kTierReported << 16);
   }
 }
 
@@ -1068,6 +1318,7 @@ static int stb_pick_e(uint32_t top_k) {
 
 #define STB_SHADOW_SCAN_U 4     // 4 rows x 4 LDG.128 per lane in flight = the f32 path's 2 x 8
 #define STB_Q8_SCAN_U 8         // 8 rows x 2 LDG.128
+#define STB_Q4_SCAN_U 16        // 16 rows x 1 LDG.128: 128 KiB in flight per SM at 2 CTAs, as q8
 
 // STB_SCAN_CTAS_PER_SM (tuning aid): resident CTAs per SM the top-k grid is sized for
 // (default: what the occupancy calculator allows, 2 with the 128-register budget).
@@ -1083,7 +1334,7 @@ static int stb_scan_ctas_per_sm_override() {
 
 template <int E, int RANGES, int SRC = 0, int EF = E>
 static int stb_launch_topk_t(stb_ctx *ctx, const TopkArgs &a_in, bool overlapped) {
-  constexpr int kU = SRC == 2 ? STB_Q8_SCAN_U : (SRC == 1 ? STB_SHADOW_SCAN_U : STB_SCAN_U);
+  constexpr int kU = SRC == 3 ? STB_Q4_SCAN_U : SRC == 2 ? STB_Q8_SCAN_U : (SRC == 1 ? STB_SHADOW_SCAN_U : STB_SCAN_U);
   auto kern = stb_scan_topk_kernel<E, kU, RANGES, SRC, EF>;
   int occ = 0;
   STB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, STB_SCAN_THREADS, 0));
@@ -1143,6 +1394,8 @@ static int stb_launch_topk_r(stb_ctx *ctx, const TopkArgs &a, int tier, uint32_t
   const int e = stb_pick_e(top_k);
   // q8: 32-key lists below the root, 128 candidates re-ranked at the root (see stb_scan_q8)
   if (tier == STB_TIER_Q8) return stb_launch_topk_t<1, RANGES, 2, 4>(ctx, a, ov);
+  // coarse + q8: 64-key warp lists by the 4-bit bound, re-scored with q8 in the CTA; 32-key lists above
+  if (tier == STB_TIER_Q4Q8) return stb_launch_topk_t<1, RANGES, 3, 4>(ctx, a, ov);
   if (tier == STB_TIER_H16) {
     switch (e) {
       case 1: return stb_launch_topk_t<1, RANGES, 1>(ctx, a, ov);
@@ -1181,7 +1434,10 @@ int stb_launch_scan_topk(stb_ctx *ctx, const stb_corpus *c, int tier, const floa
   a.shadow = c->shadow;
   a.q8 = c->q8;
   a.q8_scale = c->q8_scale;
+  a.q4 = c->q4;
+  a.q4_sr = c->q4_sr;
   if (tier == STB_TIER_Q8 && (top_k > STB_Q8_MAX_K || !c->q8)) { stb_set_error("scan_topk: q8 tier unavailable"); return STB_ERR_STATE; }
+  if (tier == STB_TIER_Q4Q8 && (top_k > STB_Q8_MAX_K || !c->q8 || !c->q4)) { stb_set_error("scan_topk: coarse q8 stage unavailable"); return STB_ERR_STATE; }
   if (tier == STB_TIER_H16 && !c->shadow) { stb_set_error("scan_topk: h16 tier unavailable"); return STB_ERR_STATE; }
   return n_ranges > 0 ? stb_launch_topk_r<1>(ctx, a, tier, top_k, overlapped) : stb_launch_topk_r<0>(ctx, a, tier, top_k, overlapped);
 }
