@@ -341,6 +341,10 @@ int stb_ctx_counters(const stb_ctx *ctx, uint64_t *kernel_launches,
 /* Consistency check of K1's dynamic tile schedule (synchronises): the device-side ticket counter
  * must equal the value the host booked over all launches so far; STB_ERR_STATE otherwise. */
 int stb_debug_ticket_check(stb_ctx *ctx, uint64_t *device_value, uint64_t *host_value);
+/* Tuning aid: K1's scan front, the virtual row at which the next ticketed top-k launch starts its
+ * wrapped scan (any value is correct; consecutive scans share HBM traffic by starting where the
+ * running one is).  set != 0 stores *value, else reads it into *value.  Synchronises. */
+int stb_debug_scan_front(stb_ctx *ctx, int set, uint64_t *value);
 /* Tuning aid: phase timestamps (ns, %globaltimer) of the last K1 launch; only filled by
  * libraries built with -DSTB_TAIL_TIMING.  reset=1 arms, reset=0 reads 8 values:
  * [0] first CTA start, [1] last scan end, [2] last CTA merge end, [3] final ticket,

@@ -27,7 +27,7 @@ SYMBOLS = [
     "stb_xchg_create", "stb_xchg_destroy", "stb_xchg_local_handle",
     "stb_xchg_connect", "stb_xchg_connect_local", "stb_search_topk_xchg", "stb_search_xchg", "stb_search_many", "stb_xchg_create_batch", "stb_search_batch_xchg_dev", "stb_ivfpq_build",
     "stb_ivfpq_destroy", "stb_ivfpq_stats", "stb_ivfpq_search", "stb_ivfpq_search_dev", "stb_hits_merge_dev", "stb_hits_merge_batch_dev", "stb_hits_merge", "stb_fnv1a64", "stb_line_id", "stb_line_ids",
-    "stb_ctx_counters", "stb_debug_ticket_check", "stb_debug_timestamps", "stb_debug_batch_gemm", "stb_debug_batch_params",
+    "stb_ctx_counters", "stb_debug_ticket_check", "stb_debug_scan_front", "stb_debug_timestamps", "stb_debug_batch_gemm", "stb_debug_batch_params",
 ]
 
 
@@ -113,6 +113,7 @@ def lib() -> C.CDLL:
     L.stb_ctx_counters.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
     L.stb_debug_timestamps.argtypes = [vp, i32, vp]
     L.stb_debug_ticket_check.argtypes = [vp, C.POINTER(u64), C.POINTER(u64)]
+    L.stb_debug_scan_front.argtypes = [vp, i32, C.POINTER(u64)]
     L.stb_debug_batch_gemm.argtypes = [vp, vp, u32, vp, u64, vp, vp]
     L.stb_debug_batch_params.argtypes = [C.POINTER(C.c_int), C.POINTER(C.c_double)]
     for name in SYMBOLS:
@@ -201,6 +202,12 @@ class Context:
         a, b = u64(0), u64(0)
         _check(lib().stb_debug_ticket_check(self._h, C.byref(a), C.byref(b)))
         return int(a.value), int(b.value)
+
+    def scan_front(self, value: int | None = None) -> int:
+        """stb_debug_scan_front: sets K1's scan front to `value` (a virtual row) if given; returns it."""
+        v = u64(0 if value is None else value)
+        _check(lib().stb_debug_scan_front(self._h, 0 if value is None else 1, C.byref(v)))
+        return int(v.value)
 
     # -- K4 ------------------------------------------------------------------
     def hits_merge(self, lists: np.ndarray, top_k: int) -> np.ndarray:

@@ -111,11 +111,13 @@ int stb_ctx_create(int device, void *cuda_stream, stb_ctx **out) {
     one = 0;
     if ((rc = dev_reserve(&c->hist_dev, &one, 4096)) != STB_OK) goto fail;
     one = 0;
-    if ((rc = dev_reserve(&c->tickets, &one, STB_TICKET_SLOTS)) != STB_OK) goto fail;
+    if ((rc = dev_reserve(&c->tickets, &one, 2 * STB_TICKET_SLOTS + 1)) != STB_OK) goto fail;
+    c->scan_start = c->tickets + STB_TICKET_SLOTS;
+    c->scan_front = c->scan_start + STB_TICKET_SLOTS;
   }
   if ((rc = dev_reserve(&c->hits_dev, &c->hits_cap, 1024)) != STB_OK) goto fail;
   if (cudaMemset(c->counters, 0, c->counters_cap * sizeof(unsigned int)) != cudaSuccess ||
-      cudaMemset(c->tickets, 0, STB_TICKET_SLOTS * sizeof(unsigned long long)) != cudaSuccess ||
+      cudaMemset(c->tickets, 0, (2 * STB_TICKET_SLOTS + 1) * sizeof(unsigned long long)) != cudaSuccess ||
       cudaMemset(c->err_flag, 0, sizeof(int)) != cudaSuccess ||
       cudaMallocHost((void **)&c->q_pin, STB_D * sizeof(float)) != cudaSuccess ||
       cudaMallocHost((void **)&c->status_pin, 8 * sizeof(uint32_t)) != cudaSuccess ||
@@ -195,6 +197,18 @@ int stb_debug_ticket_check(stb_ctx *ctx, uint64_t *device_value, uint64_t *host_
   if (device_value) *device_value = dsum;          // sums over the counter ring
   if (host_value) *host_value = hsum;
   if (bad >= 0) { stb_set_error("ticket counter %d is %llu, host expects %llu", bad, v[bad], ctx->ticket_next[bad]); return STB_ERR_STATE; }
+  return STB_OK;
+}
+
+int stb_debug_scan_front(stb_ctx *ctx, int set, uint64_t *value) {
+  int rc = ctx_use(ctx);
+  if (rc) return rc;
+  if (!value) { stb_set_error("scan_front: null value"); return STB_ERR_ARG; }
+  unsigned long long v = *value;
+  STB_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (set) STB_CUDA(cudaMemcpy(ctx->scan_front, &v, sizeof(v), cudaMemcpyHostToDevice));
+  else STB_CUDA(cudaMemcpy(&v, ctx->scan_front, sizeof(v), cudaMemcpyDeviceToHost));
+  *value = v;
   return STB_OK;
 }
 
@@ -438,9 +452,6 @@ static int stb_env_max_tier() {
   if (e[0] == 'h') return STB_TIER_H16;
   return STB_TIER_Q8;
 }
-// STB_SCAN_OVERLAP=1 (opt-in until timed on hardware): the asynchronous entry points (stb_search_topk_dev,
-// stb_search_topk_xchg, stb_search_many) use the overlapped launch mode (one CTA per SM, dependent released
-// at kernel start); default: they launch like the synchronous ones (full grid, dependent released after the scan).
 // STB_Q8_COARSE=0: no 4-bit coarse stage in front of the q8 scan.  Read per call like STB_SCAN_TIER, so
 // one process can compare the two; results are identical either way.
 static bool stb_env_coarse() {
@@ -451,10 +462,6 @@ static bool stb_env_coarse() {
 static bool stage_keeps_failing(uint32_t tries, uint32_t proven) { return tries >= 8 && 2 * proven < tries; }
 static bool coarse_usable(const stb_corpus *c) {
   return stb_env_coarse() && c->q4 && !stage_keeps_failing(c->coarse_tries, c->coarse_proven);
-}
-static bool stb_env_overlap() {
-  const char *e = getenv("STB_SCAN_OVERLAP");
-  return e && e[0] == '1';
 }
 static bool stb_env_direct_out() {
   const char *e = getenv("STB_DIRECT_OUT");
@@ -746,7 +753,7 @@ int stb_search_topk_dev(stb_ctx *ctx, const stb_corpus *corpus, const float *q_d
   // builds one: stb_corpus_prepare does); status[1] says whether the result is proven, the
   // caller's fallback is unchanged
   return stb_launch_scan_topk(ctx, corpus, best_built_tier(corpus, top_k), q_dev, top_k, nullptr, 0, corpus->n,
-                              out_hits_dev, out_status_dev, nullptr, stb_env_overlap());
+                              out_hits_dev, out_status_dev, nullptr, /*overlapped=*/true);
 }
 
 // ------------------------------------------------------------ peer-memory exchange ---
@@ -885,7 +892,7 @@ static int search_topk_xchg_impl(stb_ctx *ctx, const stb_corpus *corpus, const f
 
 int stb_search_topk_xchg(stb_ctx *ctx, const stb_corpus *corpus, const float *q_dev, uint32_t top_k,
                          stb_xchg *x, stb_hit *out_hits_dev, uint32_t *out_status_dev) {
-  return search_topk_xchg_impl(ctx, corpus, q_dev, top_k, x, out_hits_dev, out_status_dev, stb_env_overlap());
+  return search_topk_xchg_impl(ctx, corpus, q_dev, top_k, x, out_hits_dev, out_status_dev, /*overlapped=*/false);
 }
 
 // ----------------------------------------------------------------- K2 batched search ---
@@ -1272,9 +1279,9 @@ int stb_search_many(stb_ctx *ctx, const stb_corpus *corpus, const float *q, uint
   for (uint32_t i = 0; i < nq; ++i) {
     stb_hit *oh = ctx->hits_pin + (size_t)i * top_k;
     uint32_t *os = ctx->many_status_pin + 4 * (size_t)i;
-    if (x) rc = search_topk_xchg_impl(ctx, corpus, ctx->bq_dev + (size_t)i * STB_D, top_k, x, oh, os, nq > 1 && stb_env_overlap());
+    if (x) rc = search_topk_xchg_impl(ctx, corpus, ctx->bq_dev + (size_t)i * STB_D, top_k, x, oh, os, /*overlapped=*/false);
     else rc = stb_launch_scan_topk(ctx, corpus, tier, ctx->bq_dev + (size_t)i * STB_D, top_k, nullptr, 0, corpus->n, oh, os, nullptr,
-                                   nq > 1 && stb_env_overlap());
+                                   /*overlapped=*/nq > 1);
     if (rc != STB_OK) { cudaStreamSynchronize(ctx->stream); return rc; }
   }
   STB_CUDA(cudaStreamSynchronize(ctx->stream));

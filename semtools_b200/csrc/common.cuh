@@ -78,12 +78,13 @@ struct stb_ctx {
   unsigned int *counters;   // tree arrival counters (zeroed; kernels re-zero)
   size_t counters_cap;
   // K1 tile-ticket counters (monotonic; scan_topk.cu: stb_for_each_tile).  A ring of STB_TICKET_SLOTS
-  // counters, one per launch in turn: with the overlapped launch mode two consecutive scans run
-  // concurrently and must not draw from the same counter.
-  unsigned long long *tickets;
+  // counters, one per launch in turn: two consecutive scans may run concurrently and must not draw
+  // from the same counter.
+  unsigned long long *tickets;         // [STB_TICKET_SLOTS] counters, then the words below
+  unsigned long long *scan_start;      // [STB_TICKET_SLOTS] per slot: (launch seq << 32) | start tile
+  unsigned long long *scan_front;      // [1] a virtual row a running scan reached (synchronized scans)
   unsigned long long ticket_next[8];   // per slot: its value when the next launch using it starts
   unsigned long long topk_launches;    // picks the slot
-  bool ticket_ring;                    // set by the first overlapped launch; until then every launch uses slot 0
   float *q_dev;             // 256 f32 staging for host queries
   stb_hit *hits_dev;        // result hits (top-k path)
   size_t hits_cap;

@@ -54,11 +54,15 @@ struct ScanArgs {
   const uint64_t *rbegin;    // [n_ranges]   local first row of each range
   uint32_t n_ranges;
   // dynamic tile schedule (top-k kernel; null = static warp-strided schedule):
-  unsigned long long *tickets;   // monotonic counter shared by every launch of the context
+  unsigned long long *tickets;   // this launch's counter of the context's ring (monotonic)
   unsigned long long t_base;     // its value when this launch starts (host-tracked)
   uint64_t t_bulk;               // tickets [0, t_bulk) cover STB_TICKET_TILES tiles each, later ones one tile
+  unsigned long long *start;     // this launch's ring word: (seq << 32) | first tile, once published
+  unsigned long long *front;     // the context's scan front: a virtual row some running scan reached
+  uint32_t seq;                  // launch number (never 0): tells this launch's start from a stale one
 };
 #define STB_TICKET_TILES 4
+#define STB_FRONT_EVERY 64       // tickets per store to the scan front
 
 // ---- tile schedule + row map shared by the three scans -----------------------------------
 // RANGES == 0: whole shard, tiles are warp-strided (the grid streams one contiguous window).
@@ -75,8 +79,32 @@ struct ScanArgs {
 // K'=128) on every pipelined query.  With tickets a late CTA simply finds less work.
 // Every warp makes exactly one failing draw, so a launch advances the counter by
 // n_tickets + total_warps -- the host tracks the base of the next launch with that.
+// Synchronized scans: a launch does not start at tile 0 but at the tile s where some running scan of the
+// context currently is, and wraps around: ticket t covers tiles (s + first_tile(t) + i) mod n_tiles.  Two
+// co-resident grids (overlapped launches) then stream the same lines at the same time, so each line comes
+// from HBM once for both; a launch that follows a finished one starts on the lines still in L2.  Warps
+// store the first virtual row of every STB_FRONT_EVERY-th ticket to args.front; any value is correct,
+// only the sharing depends on it.  body(tile, restart): restart is set at a ticket's first tile and at
+// the wrap to tile 0 (the row-ranges map walks forward only).
+__device__ __forceinline__ void stb_st_release_gpu(unsigned long long *p, unsigned long long v) {
+  asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ unsigned long long stb_ld_acquire_gpu(const unsigned long long *p) {
+  unsigned long long v;
+  asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ void stb_st_relaxed_gpu(unsigned long long *p, unsigned long long v) {
+  asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ unsigned long long stb_ld_relaxed_gpu(const unsigned long long *p) {
+  unsigned long long v;
+  asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+
 template <int RANGES, int WB, class Body>
-__device__ __forceinline__ void stb_for_each_tile(const ScanArgs &args, uint64_t n_tiles, Body &&body) {
+__device__ __forceinline__ void stb_for_each_tile(const ScanArgs &args, uint64_t n_tiles, uint64_t tile_rows, Body &&body) {
   if (args.tickets) {
     // The next ticket is drawn BEFORE the current one is processed, so the atomic's L2 round trip
     // (~1 us under load) overlaps a ticket's worth of loads instead of stalling the warp 4-6 times per
@@ -92,13 +120,36 @@ __device__ __forceinline__ void stb_for_each_tile(const ScanArgs &args, uint64_t
       return t < args.t_bulk ? t * STB_TICKET_TILES : args.t_bulk * STB_TICKET_TILES + (t - args.t_bulk);
     };
     unsigned long long cur = draw();
-    while (first_tile(cur) < n_tiles) {
+    if (first_tile(cur) >= n_tiles) return;
+    // The start tile s: the warp that drew ticket 0 reads the front and publishes s for this launch; the
+    // others wait for it.  No deadlock: a waiter depends only on a warp of its own grid, and that warp is
+    // resident (it has drawn ticket 0) and publishes before it waits on anything.  The word is tagged with
+    // the launch number, so nothing is reset between launches.
+    uint64_t s = 0;
+    if (lane == 0) {
+      if (cur == 0) {
+        s = (stb_ld_relaxed_gpu(args.front) % args.n_virtual) / tile_rows;
+        stb_st_release_gpu(args.start, ((unsigned long long)args.seq << 32) | s);
+      } else {
+        unsigned long long w;
+        while (((w = stb_ld_acquire_gpu(args.start)) >> 32) != args.seq) __nanosleep(100);
+        s = w & 0xffffffffull;
+      }
+    }
+    s = __shfl_sync(0xffffffffu, s, 0);
+    do {
       const unsigned long long nxt = draw();
       const uint64_t t0 = first_tile(cur);
       const uint64_t t1 = cur < args.t_bulk ? t0 + STB_TICKET_TILES : t0 + 1;
-      for (uint64_t tile = t0; tile < t1; ++tile) body(tile, tile == t0);
+      uint64_t tile = s + t0;
+      if (tile >= n_tiles) tile -= n_tiles;
+      if (lane == 0 && cur % STB_FRONT_EVERY == 0) stb_st_relaxed_gpu(args.front, tile * tile_rows);
+      for (uint64_t i = t0; i < t1; ++i) {
+        body(tile, i == t0 || tile == 0);
+        if (++tile == n_tiles) tile = 0;
+      }
       cur = nxt;
-    }
+    } while (first_tile(cur) < n_tiles);
     return;
   }
   const uint64_t warps_total = (uint64_t)gridDim.x * (blockDim.x >> 5);
@@ -187,7 +238,7 @@ __device__ __forceinline__ void stb_scan_rows(const ScanArgs &args, Sink &sink) 
   const uint64_t n_tiles = (args.n_virtual + tile_rows - 1) / tile_rows;
   StbRowMap<RANGES> rmap;
   rmap.restart();
-  stb_for_each_tile<RANGES, 64 / (4 * U)>(args, n_tiles, [&](uint64_t tile, bool first) {
+  stb_for_each_tile<RANGES, 64 / (4 * U)>(args, n_tiles, tile_rows, [&](uint64_t tile, bool first) {
     if (first) rmap.restart();
     float4 a[U][8];
     uint32_t row[U];
@@ -281,7 +332,7 @@ __device__ __forceinline__ void stb_scan_shadow(const ScanArgs &args, const uint
   const uint64_t n_tiles = (args.n_virtual + tile_rows - 1) / tile_rows;
   StbRowMap<RANGES> rmap;
   rmap.restart();
-  stb_for_each_tile<RANGES, 64 / (4 * U)>(args, n_tiles, [&](uint64_t tile, bool first) {
+  stb_for_each_tile<RANGES, 64 / (4 * U)>(args, n_tiles, tile_rows, [&](uint64_t tile, bool first) {
     if (first) rmap.restart();
     uint4 a[U][4];
     uint32_t row[U];
@@ -429,7 +480,7 @@ __device__ __forceinline__ void stb_scan_q8(const ScanArgs &args, const uint8_t 
   const uint64_t n_tiles = (args.n_virtual + tile_rows - 1) / tile_rows;
   StbRowMap<RANGES> rmap;
   rmap.restart();
-  stb_for_each_tile<RANGES, 2>(args, n_tiles, [&](uint64_t tile, bool first) {
+  stb_for_each_tile<RANGES, 2>(args, n_tiles, tile_rows, [&](uint64_t tile, bool first) {
     if (first) rmap.restart();
     uint4 a[U][2];
     float sc_row[U];
@@ -463,13 +514,20 @@ __device__ __forceinline__ void stb_scan_q8(const ScanArgs &args, const uint8_t 
   });
 }
 
+// dp4a with unsigned bytes in a and signed bytes in b (PTX dp4a.u32.s32)
+__device__ __forceinline__ int stb_dp4a_us(uint32_t a, uint32_t b, int c) {
+  int d;
+  asm("dp4a.u32.s32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(c));
+  return d;
+}
+
 // Coarse pass in front of the q8 tier ("q4"): a 4-bit copy, 128 B of codes + (s4, r) per row = 136 B.
 // Row model (stb_q4_build_kernel): x~_i = s4 * (c_i - 7.5), c_i in [0, 15] (16 mid-rise levels) on the
 // fp32-normalised row x^, with s4 picked per row to minimise r = ||x^ - x~||_2, stored rounded up.
 // Byte b of the row's 32-bit word l holds c[8l+b] in its low nibble and c[8l+4+b] in its high one, so
 // lane j of a row group reads one 16-byte chunk = elements 32j .. 32j+31, and the query, quantised per
 // call to int8 (q8_i = rint(q^_i * S8), S8 = 127 / max|q^_i|), lines up byte for byte with the two
-// nibble planes: two masks, one shift and two dp4a per word, exact in int32.  With q~ = q8 / S8 and
+// nibble planes: two masks and two dp4a per word, exact in int32.  With q~ = q8 / S8 and
 // f = q^ - q~, Cauchy-Schwarz gives for the exact cosine c = q^ . x^:
 //     c = q~ . x~ + q~ . (x^ - x~) + f . x^  <=  q~ . x~ + r (1 + ||f||) + ||f||
 //     q~ . x~ = s4 * (2 dot - 15 sum(q8)) / (2 S8)          (integer part exact)
@@ -527,41 +585,74 @@ __device__ __forceinline__ void stb_scan_q4(const ScanArgs &args, const uint8_t 
   const uint64_t n_tiles = (args.n_virtual + tile_rows - 1) / tile_rows;
   StbRowMap<RANGES> rmap;
   rmap.restart();
-  stb_for_each_tile<RANGES, 1>(args, n_tiles, [&](uint64_t tile, bool first) {
+  stb_for_each_tile<RANGES, 1>(args, n_tiles, tile_rows, [&](uint64_t tile, bool first) {
     if (first) rmap.restart();
     uint4 a[U];
     uint32_t own_row[U / 8];   // the rows this lane hands to the sink: u = j + 8h
+    const uint64_t v0 = tile * tile_rows;
+    const bool full = RANGES == 0 && v0 + tile_rows <= args.n_virtual;   // warp-uniform
+    if (full) {
+      // every row exists and is its own local row: one base address, the rows at immediate offsets
+      const float4 *p = reinterpret_cast<const float4 *>(q4 + (size_t)(v0 + g) * 128 + (size_t)j * 16);
 #pragma unroll
-    for (int u = 0; u < U; ++u) {
-      const uint64_t v = tile * tile_rows + (uint64_t)(u * 4 + g);
-      const uint64_t vc = v < args.n_virtual ? v : (args.n_virtual - 1);
-      const uint32_t row = rmap.map(args, vc);
-      const float4 t = stb_ld_stream(reinterpret_cast<const float4 *>(q4 + (size_t)row * 128 + (size_t)j * 16));
-      a[u] = make_uint4(__float_as_uint(t.x), __float_as_uint(t.y), __float_as_uint(t.z), __float_as_uint(t.w));
-      if ((u & 7) == j) own_row[u >> 3] = row;
+      for (int u = 0; u < U; ++u) {
+        const float4 t = stb_ld_stream(p + u * 32);   // + 4 rows of 128 B
+        a[u] = make_uint4(__float_as_uint(t.x), __float_as_uint(t.y), __float_as_uint(t.z), __float_as_uint(t.w));
+      }
+#pragma unroll
+      for (int h = 0; h < U / 8; ++h) own_row[h] = (uint32_t)(v0 + (uint64_t)((8 * h + j) * 4 + g));
+    } else {
+#pragma unroll
+      for (int u = 0; u < U; ++u) {
+        const uint64_t v = v0 + (uint64_t)(u * 4 + g);
+        const uint64_t vc = v < args.n_virtual ? v : (args.n_virtual - 1);
+        const uint32_t row = rmap.map(args, vc);
+        const float4 t = stb_ld_stream(reinterpret_cast<const float4 *>(q4 + (size_t)row * 128 + (size_t)j * 16));
+        a[u] = make_uint4(__float_as_uint(t.x), __float_as_uint(t.y), __float_as_uint(t.z), __float_as_uint(t.w));
+        if ((u & 7) == j) own_row[u >> 3] = row;
+      }
     }
 #pragma unroll
     for (int h = 0; h < U / 8; ++h) {
       const float2 sr = __ldg(q4_sr + own_row[h]);
-      int own_dot = 0;
+      // x[uu] = 16 * this lane's part of the dot of row u = 8h + uu: the high nibbles are dotted in place
+      // (w & 0xF0F0F0F0 = 16 * code, unsigned bytes against the signed query bytes), so no shift per word
+      int x[8];
 #pragma unroll
       for (int uu = 0; uu < 8; ++uu) {
         const uint4 &w = a[8 * h + uu];
         const uint32_t ww[4] = {w.x, w.y, w.z, w.w};
-        int d = 0;
+        int dl = 0, dh = 0;
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-          d = __dp4a((int)(ww[i] & 0x0f0f0f0fu), (int)qw[2 * i], d);
-          d = __dp4a((int)((ww[i] >> 4) & 0x0f0f0f0fu), (int)qw[2 * i + 1], d);
+          dl = __dp4a((int)(ww[i] & 0x0f0f0f0fu), (int)qw[2 * i], dl);
+          dh = stb_dp4a_us(ww[i] & 0xf0f0f0f0u, qw[2 * i + 1], dh);
         }
-        d += __shfl_xor_sync(0xffffffffu, d, 4);
-        d += __shfl_xor_sync(0xffffffffu, d, 2);
-        d += __shfl_xor_sync(0xffffffffu, d, 1);
-        if (uu == j) own_dot = d;
+        x[uu] = dh + 16 * dl;
       }
-      const uint64_t v = tile * tile_rows + (uint64_t)((8 * h + j) * 4 + g);
+      // transpose-reduce over the 8 lanes of the group by recursive halving: at each step a lane keeps the
+      // half of its rows whose index agrees with j on that bit and adds its partner's copy of the same rows,
+      // so lane j ends with the full sum of row uu = j (7 shuffles for 8 rows instead of 24)
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const bool hi = j & 4;
+        const int keep = hi ? x[i + 4] : x[i], send = hi ? x[i] : x[i + 4];
+        x[i] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
+      }
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        const bool hi = j & 2;
+        const int keep = hi ? x[i + 2] : x[i], send = hi ? x[i] : x[i + 2];
+        x[i] = keep + __shfl_xor_sync(0xffffffffu, send, 2);
+      }
+      {
+        const bool hi = j & 1;
+        const int keep = hi ? x[1] : x[0], send = hi ? x[0] : x[1];
+        x[0] = keep + __shfl_xor_sync(0xffffffffu, send, 1);
+      }
+      const int own_dot = x[0] >> 4;                      // exact: x[0] = 16 * dot
       float s = q_unusable ? CUDART_INF_F : fmaf(sr.x * coef, (float)(2 * own_dot - qsum15), fmaf(sr.y, r_mul, slack));
-      if (v >= args.n_virtual) s = -CUDART_INF_F;
+      if (!full && v0 + (uint64_t)((8 * h + j) * 4 + g) >= args.n_virtual) s = -CUDART_INF_F;
       sink.template consume<32>(s, own_row[h]);
     }
   });
@@ -1363,14 +1454,16 @@ static int stb_launch_topk_t(stb_ctx *ctx, const TopkArgs &a_in, bool overlapped
     const uint64_t single = std::min<uint64_t>(tiles, 2 * warps_total);
     a.scan.t_bulk = (tiles - single) / STB_TICKET_TILES;
     const uint64_t n_tickets = a.scan.t_bulk + (tiles - a.scan.t_bulk * STB_TICKET_TILES);
-    // one counter serves back-to-back launches (a grid starts drawing only after its predecessor's scan, the
-    // validated default); the ring is needed -- and used -- from the first overlapped launch on, when two
-    // consecutive scans co-run (at most ~3 grids are ever in flight)
-    if (overlapped) ctx->ticket_ring = true;
-    const int slot = ctx->ticket_ring ? (int)(ctx->topk_launches++ % STB_TICKET_SLOTS) : 0;
+    // consecutive launches draw from different counters of the ring: two overlapped scans co-run, and a
+    // straggler warp of a finished scan must not take a ticket of the next one (at most ~3 grids are ever
+    // in flight, far fewer than STB_TICKET_SLOTS)
+    const int slot = (int)(ctx->topk_launches++ % STB_TICKET_SLOTS);
     a.scan.tickets = ctx->tickets + slot;
     a.scan.t_base = ctx->ticket_next[slot];
     ctx->ticket_next[slot] += n_tickets + warps_total;
+    a.scan.start = ctx->scan_start + slot;
+    a.scan.front = ctx->scan_front;
+    a.scan.seq = (uint32_t)ctx->topk_launches;   // the slot's previous launch had seq - STB_TICKET_SLOTS; never 0 mod 2^32 twice in a row
   }
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
@@ -1421,7 +1514,7 @@ int stb_launch_scan_topk(stb_ctx *ctx, const stb_corpus *c, int tier, const floa
   a.scan.vstart = ranges_dev;
   a.scan.rbegin = ranges_dev ? ranges_dev + (n_ranges + 1) : nullptr;
   a.scan.n_ranges = n_ranges;
-  a.scan.tickets = nullptr; a.scan.t_base = 0; a.scan.t_bulk = 0;
+  a.scan.tickets = nullptr; a.scan.t_base = 0; a.scan.t_bulk = 0; a.scan.start = a.scan.front = nullptr; a.scan.seq = 0;
   a.row_base = c->row_base;
   a.keys = ctx->block_keys;
   a.counters = ctx->counters;
@@ -1496,7 +1589,7 @@ int stb_launch_scan_collect(stb_ctx *ctx, const stb_corpus *c, int tier,
   a.scan.vstart = ranges_dev;
   a.scan.rbegin = ranges_dev ? ranges_dev + (n_ranges + 1) : nullptr;
   a.scan.n_ranges = n_ranges;
-  a.scan.tickets = nullptr; a.scan.t_base = 0; a.scan.t_bulk = 0;
+  a.scan.tickets = nullptr; a.scan.t_base = 0; a.scan.t_bulk = 0; a.scan.start = a.scan.front = nullptr; a.scan.seq = 0;
   a.cos_floor = cos_floor;
   a.out = ctx->collect_rows;
   a.count = ctx->collect_count;
@@ -1561,7 +1654,7 @@ int stb_launch_scan_hist(stb_ctx *ctx, const stb_corpus *c, int tier, const floa
   a.vstart = ranges_dev;
   a.rbegin = ranges_dev ? ranges_dev + (n_ranges + 1) : nullptr;
   a.n_ranges = n_ranges;
-  a.tickets = nullptr; a.t_base = 0; a.t_bulk = 0;
+  a.tickets = nullptr; a.t_base = 0; a.t_bulk = 0; a.start = a.front = nullptr; a.seq = 0;
   STB_CUDA(cudaMemsetAsync(hist_dev, 0, STB_HIST_BINS * sizeof(unsigned int), ctx->stream));
   const int u = tier == STB_TIER_Q8 ? STB_Q8_SCAN_U : STB_SCAN_U;
   uint64_t tiles = (n_virtual + 4 * u - 1) / (4 * u);
